@@ -1,4 +1,4 @@
-"""Drive the UNMODIFIED reference (baseline/_ref, or /root/reference in the build container) the way
+"""Drive the UNMODIFIED reference (compiled into oracle/_ref by oracle/fetch_ref.py) the way
 experiment/run.py:38-49 does: setup_architecture -> maybe_cuda -> setup_opt -> agents[...](model, opt,
 params) -> train_learner(uint8 NHWC array, labels).  Import recipe = SURVEY.md Appendix B: three stub
 modules that are not on the arithmetic path (matplotlib, skimage, kornia -- none is installed here and
@@ -27,10 +27,8 @@ TRICK = {'labels_trick': False, 'kd_trick': False, 'separated_softmax': False, '
 
 
 def locate():
-    for p in (os.path.join(HERE, '_ref'), '/root/reference'):
-        if os.path.exists(os.path.join(p, 'utils', 'name_match.py')):
-            return p
-    return None
+    p = os.path.join(os.path.dirname(HERE), 'oracle', '_ref')
+    return p if os.path.exists(os.path.join(p, 'utils', 'name_match.pyc')) else None
 
 
 def import_reference(path=None):
@@ -38,7 +36,7 @@ def import_reference(path=None):
     import torch.nn as nn
     path = path or locate()
     if path is None:
-        raise RuntimeError('no reference tree: run `python baseline/fetch_ref.py` in the build container')
+        raise RuntimeError('no reference build: run `python oracle/fetch_ref.py <reference checkout>`')
     if path not in sys.path:
         sys.path.insert(0, path)
     if 'kornia.augmentation' not in sys.modules:

@@ -2,7 +2,7 @@
 """Replay-step throughput bench (BASELINE.json metric: replay-step images/sec, ASER+SCR,
 Reduced-ResNet18, CIFAR-100 shapes, mem_size 5000).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 One *step* = one ER+ASER replay step (BASELINE config 3: asvm, k=3, n_smp_cls 1.5, 10 stream + 10
@@ -16,7 +16,10 @@ images per step.  Inputs are synthetic (uniform images, uniform labels), weights
   N > 1  data-parallel stream shards: every rank runs its own stream shard and memory, gradients are
          averaged with one NCCL all-reduce of the flat gradient arena per optimizer step (weak scaling)
   --impl reference   the reference's algorithm on the host CPU cores (oracle/replay_step.py, the
-         restatement pinned against the reference's agents; /root/reference does not travel to the box)
+         restatement pinned against the reference's agents) when oracle/_ref is absent
+  --dump-outputs DIR   after the timed steps, write what the last device-resident step left a caller
+         (both losses, weights, BN statistics, memory labels, a seeded sample of memory images) as
+         DIR/<name>.npy, so that two builds can be compared output for output on identical inputs
 """
 import argparse
 import json
@@ -31,6 +34,7 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True           # the tree may be read-only: nothing is written into it
 
 WORKLOAD = ('ER+ASER replay step (asvm,k=3,n_smp_cls=1.5,10+10 imgs) + SCR replay step '
             '(SupCon T=0.07,mlp head,10+100 imgs x 2 views), CIFAR-100 shapes, mem_size 5000, batch 10')
@@ -220,6 +224,8 @@ def run_ours(args, rank, world):
     log('rank %d: learners built' % rank)
     ms_dev, launches, clocks, wall, stats = timed(False)
     log('rank %d: device-resident pass %.2f ms/step' % (rank, ms_dev / args.steps))
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {'aser': aser, 'scr': scr})
     ms_e2e, _, _, _, stats_e2e = timed(True)
     log('rank %d: end-to-end pass %.2f ms/step' % (rank, ms_e2e / args.steps))
     if rank != 0:
@@ -254,6 +260,27 @@ def run_ours(args, rank, world):
         line['roofline'] = prof['roofline']
         line['kernel_ms_per_step'] = prof['classes']
     return line
+
+
+def dump_outputs(out_dir, learners, n_img_rows=256):
+    """What the last timed step left a caller of replay_step: its loss, the weights and BatchNorm running
+    statistics of the model, the memory's labels and a fixed, seeded sample of the memory's image rows
+    (the whole memory is 61 MB per learner).  float32 arrays as computed; labels and losses as float64."""
+    import torch
+    torch.cuda.synchronize()
+    os.makedirs(out_dir, exist_ok=True)
+    for name, L in learners.items():
+        buf = L.buffer
+        rows = np.sort(np.random.RandomState(0).choice(buf.buffer_img.shape[0], n_img_rows, replace=False))
+        arrays = {'loss': np.array([float(L.last_loss)], dtype=np.float64),
+                  'params': L.engine.state.params.cpu().numpy(),
+                  'bn_stats': L.engine.state.bn_stats.cpu().numpy(),
+                  'buffer_label': buf.buffer_label.cpu().numpy().astype(np.float64),
+                  'buffer_img_rows': rows.astype(np.float64),
+                  'buffer_img_sample': buf.buffer_img[torch.from_numpy(rows).to(buf.buffer_img.device)].cpu().numpy()}
+        for k, a in arrays.items():
+            np.save(os.path.join(out_dir, '%s_%s.npy' % (name, k)), a)
+    log('outputs of the last timed step written to %s' % out_dir)
 
 
 def profile_step(step_fn, i):
@@ -452,7 +479,7 @@ T0 = time.perf_counter()
 
 
 def run_reference_harness(device, steps, warmup, timeout_s=600):
-    """The UNMODIFIED reference agents (baseline/_ref, materialised by baseline/fetch_ref.py) through
+    """The UNMODIFIED reference agents (oracle/_ref, compiled by oracle/fetch_ref.py) through
     baseline/ref_harness.py in a subprocess: --device cpu hides the GPUs so that every
     torch.cuda.is_available() gate of the reference is off; --device cuda is the reference's own
     single-GPU PyTorch path (cudnn.deterministic as general_main.py:15-18).  None if the tree is absent."""
@@ -486,7 +513,7 @@ def run_reference_harness(device, steps, warmup, timeout_s=600):
 
 def run_reference(args, steps, warmup, budget_s=30.0):
     """The reference's replay step on the host cores.  Preferred: the unmodified reference itself
-    (kind "reference"); without baseline/_ref: oracle/replay_step.py, the restatement pinned against it
+    (kind "reference"); without oracle/_ref: oracle/replay_step.py, the restatement pinned against it
     (kind "port").  Each step is one ER+ASER step and one SCR step like the CUDA arm."""
     h = run_reference_harness('cpu', steps, warmup)
     if h is not None:
@@ -541,6 +568,7 @@ def main():
     ap.add_argument('--impl', default='ours', choices=['ours', 'reference'])
     ap.add_argument('--no-cpu-baseline', action='store_true')
     ap.add_argument('--workload', default='replay', choices=['replay', 'knn_sweep'])
+    ap.add_argument('--dump-outputs', metavar='DIR', default=None)
     args = ap.parse_args()
     args.warmup = max(args.warmup, 3) if args.impl == 'ours' else args.warmup
     rank = int(os.environ.get('RANK', 0))
@@ -550,8 +578,8 @@ def main():
         if rank != 0:
             return 0
         os.environ['CUDA_VISIBLE_DEVICES'] = ''                      # the CPU arm never touches a GPU
-        steps, warmup = min(args.steps, 40), max(1, min(args.warmup, 2))   # ~0.4 s per step pair on 16 cores
-        r = run_reference(args, steps, warmup, budget_s=90.0)
+        steps, warmup = args.steps, max(1, args.warmup)
+        r = run_reference(args, steps, warmup, budget_s=float('inf'))
         steps = r['steps']
         line = {'impl': 'reference', 'metric': 'replay-step images/sec (ASER+SCR, ResNet18, CIFAR100)',
                 'value': r['value'], 'unit': 'stream images/s', 'n_gpus': args.gpus, 'steps': steps, 'warmup': warmup,
@@ -595,7 +623,7 @@ def main():
                 line['reference_gpu'] = {
                     'value': g['stream_images_per_s'], 'unit': 'stream images/s', 'ms_per_step': g['ms_per_step_pair'],
                     'aser_ms': g['aser_ms_per_step'], 'scr_ms': g['scr_ms_per_step'],
-                    'what': 'unmodified reference agents (baseline/_ref) on cuda:0 of this box, torch %s eager, '
+                    'what': 'unmodified reference agents (oracle/_ref) on cuda:0, torch %s eager, '
                             'cudnn.deterministic=True, benchmark=False (general_main.py:15-18), same workload, '
                             '40 steps after 5 warm-up, identity augmentation stub (kornia absent: the reference does '
                             'less work than in production)' % g['torch']}

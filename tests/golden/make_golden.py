@@ -537,10 +537,103 @@ def gen_gss():
     np.savez_compressed(os.path.join(HERE, 'gss.npz'), **out)
 
 
+# ----------------------------------------------------------------------------- parity-mode random streams
+def _digest(t):
+    import hashlib
+    return np.frombuffer(hashlib.sha256(t.contiguous().numpy().tobytes()).digest(), np.uint8)
+
+
+def gen_parity():
+    """The reference's host-side random decisions on the inputs of tests/test_parity_mode.py: class-balanced
+    sampler draws (buffer_utils.py:60-140), reservoir updates (reservoir_update.py:8-60) and the stream
+    DataLoader order (continuum/data_utils.py).  Image tensors are recorded as sha256 digests of their bytes."""
+    from continuum.data_utils import dataset_transform
+    from utils.setup_elements import transforms_match
+    from torch.utils import data
+    Ref = buffer_utils.ClassBalancedRandomSampling
+    out = {}
+
+    def sample(n, excl, seed):
+        torch.manual_seed(seed)
+        return Ref.sample(buf_x, buf_y, n, excl_indices=None if excl is None else set(excl), device='cpu')[2].numpy()
+    for n_cls, mem in [(10, 200), (100, 1000)]:
+        Ref.class_index_cache = Ref.class_num_cache = None
+        tag = 'inc%d' % n_cls
+        rs = np.random.RandomState(3)
+        labels = rs.randint(0, n_cls, mem).astype(np.int64)
+        buf_y = torch.zeros(mem, dtype=torch.int64)
+        buf_x = torch.zeros(mem, 1)
+        for s in range(0, mem, 10):
+            ny = torch.from_numpy(labels[s:s + 10])
+            Ref.update_cache(buf_y, n_cls, new_y=ny, ind=torch.arange(s, s + 10), device='cpu')
+            buf_y[s:s + 10] = ny
+        out[tag + '_keys'] = np.array(list(Ref.class_index_cache.keys()))
+        for step in range(25):
+            r1 = sample(1, None, 100 + step)
+            r2 = sample(2, r1.tolist(), 200 + step)
+            out['%s_r1_%d' % (tag, step)], out['%s_r2_%d' % (tag, step)] = r1, r2
+            slots = rs.choice(mem, 4, replace=False)
+            ny = rs.randint(0, n_cls, 4).astype(np.int64)
+            Ref.update_cache(buf_y, n_cls, new_y=torch.from_numpy(ny), ind=torch.from_numpy(slots), device='cpu')
+            buf_y[torch.from_numpy(slots)] = torch.from_numpy(ny)
+            out['%s_num_%d' % (tag, step)] = Ref.class_num_cache.numpy().copy()
+    Ref.class_index_cache = Ref.class_num_cache = None
+    rs = np.random.RandomState(4)
+    buf_y = torch.from_numpy(rs.randint(0, 20, 300).astype(np.int64))
+    buf_x = torch.zeros(300, 1)
+    Ref.update_cache(buf_y, 20)
+    out['rebuild_keys'] = np.array(list(Ref.class_index_cache.keys()))
+    for step in range(10):
+        r = sample(3, None, step)
+        out['rebuild_r_%d' % step], out['rebuild_r2_%d' % step] = r, sample(3, r.tolist(), 50 + step)
+    Ref.class_index_cache = Ref.class_num_cache = None
+
+    params = SimpleNamespace(data='cifar10', cuda=False, mem_size=50, update='random', retrieve='random',
+                             eps_mem_batch=10, buffer_tracker=False)
+    buf = SimpleNamespace(buffer_img=torch.zeros(50, 3, 32, 32), buffer_label=torch.zeros(50, dtype=torch.int64),
+                          current_index=0, n_seen_so_far=0, params=params)
+    upd = reservoir_update.Reservoir_update(params)
+    rs = np.random.RandomState(0)
+    labels, imgs, n_seen = [], [], []
+    for step in range(30):
+        x = torch.from_numpy(rs.rand(10, 3, 32, 32).astype(np.float32))
+        y = torch.from_numpy(rs.randint(0, 10, 10).astype(np.int64))
+        torch.manual_seed(step)
+        out['reservoir_ret_%d' % step] = np.array(list(upd.update(buf, x, y)), dtype=np.int64)
+        labels.append(buf.buffer_label.numpy().copy()); imgs.append(_digest(buf.buffer_img)); n_seen.append(buf.n_seen_so_far)
+    out.update(reservoir_label=np.stack(labels), reservoir_img_sha256=np.stack(imgs), reservoir_n_seen=np.array(n_seen))
+
+    rs = np.random.RandomState(1)
+    x = rs.randint(0, 256, (57, 32, 32, 3)).astype(np.uint8)
+    y = rs.randint(0, 10, 57).astype(np.int64)
+    torch.manual_seed(11)
+    loader = data.DataLoader(dataset_transform(x, y, transform=transforms_match['cifar10']), batch_size=10,
+                             shuffle=True, num_workers=0, drop_last=True)
+    batches = [(bx.clone(), by.clone()) for bx, by in loader]
+    out.update(stream_label=np.stack([by.numpy() for _, by in batches]),
+               stream_img_sha256=np.stack([_digest(bx) for bx, _ in batches]),
+               stream_img_shape=np.array(batches[0][0].shape), stream_rand_after=torch.rand(1).numpy())
+    np.savez_compressed(os.path.join(HERE, 'parity.npz'), **out)
+
+
+def gen_registry():
+    """The registry keys of utils/name_match.py and the module-level names the drop-in switch rebinds."""
+    import agents.base as base
+    import experiment.run as run
+    import utils.name_match as nm
+    out = {t: np.array(sorted(getattr(nm, t))) for t in ('agents', 'retrieve_methods', 'update_methods')}
+    out['run_agents_is_name_match_agents'] = np.bool_(run.agents is nm.agents)
+    out['patched'] = np.array(['agents.base:SupConLoss', 'utils.buffer.aser_retrieve:compute_knn_sv',
+                               'utils.buffer.aser_update:compute_knn_sv'])
+    assert all(hasattr(m, 'compute_knn_sv') for m in (aser_retrieve, aser_update)) and hasattr(base, 'SupConLoss')
+    np.savez_compressed(os.path.join(HERE, 'registry.npz'), **out)
+
+
 if __name__ == '__main__':
     only = sys.argv[2:]            # e.g. `make_golden.py /root/reference gss`: regenerate one file
     for name, fn in (('knn_sv', gen_knn_sv), ('supcon', gen_supcon), ('resnet', gen_resnet), ('aser', gen_aser),
-                     ('reservoir', gen_reservoir), ('steps', gen_steps), ('gss', gen_gss)):
+                     ('reservoir', gen_reservoir), ('steps', gen_steps), ('gss', gen_gss), ('parity', gen_parity),
+                     ('registry', gen_registry)):
         if not only or name in only:
             fn()
     for f in sorted(os.listdir(HERE)):

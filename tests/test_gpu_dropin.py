@@ -4,7 +4,7 @@ torch.optim.SGD, `b200ocl.install()` swaps the replay-path entries of the refere
 agents[...](model, opt, params).train_learner(uint8 NHWC) / .evaluate(test_loaders) run, at the BASELINE
 sizes (mem_size 5000, CIFAR-100 shapes, lr 0.1; MIR at 84x84 with mem 10000).
 
-The same seeded script is first executed with the unmodified reference (baseline/_ref, same GPU) and
+The same seeded script is first executed with the unmodified reference (oracle/_ref, same GPU) and
 recorded after every train_learner call (one replay step per call).  The b200ocl run (parity mode: no
 injected sampler choices) must then reproduce, call by call:
   * bit-exact: buffer_label, buffer_img, current_index, n_seen_so_far (= the slots retrieved / evicted),
@@ -36,7 +36,7 @@ sys.path.insert(0, os.path.join(ROOT, 'baseline'))
 import ref_harness  # noqa: E402
 
 pytestmark = [pytest.mark.gpu,
-              pytest.mark.skipif(ref_harness.locate() is None, reason='baseline/_ref missing (python baseline/fetch_ref.py)')]
+              pytest.mark.skipif(ref_harness.locate() is None, reason='oracle/_ref missing (python oracle/fetch_ref.py)')]
 
 REPORT = {}
 REPORT_ONLY = bool(os.environ.get('B200OCL_DROPIN_REPORT_ONLY'))   # diagnostics: record the errors, skip the tolerance asserts
@@ -340,5 +340,5 @@ def test_dropin_matches_reference_run(kind, n_calls, n_label, over):
 
 
 def test_reference_copy_is_unmodified():
-    import fetch_ref
+    from oracle import fetch_ref
     assert fetch_ref.verify()

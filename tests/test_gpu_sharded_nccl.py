@@ -24,7 +24,7 @@ def _free_port():
 @pytest.mark.parametrize('rows,cand,dim', [(5001, 160, 160), (20000, 1000, 512)])
 def test_sharded_knn_sv_nccl_world2(rows, cand, dim):
     if torch.cuda.device_count() < 2:
-        pytest.skip('needs 2 GPUs (run under `gpurun --gpus 2`)')
+        pytest.skip('needs 2 GPUs')
     env = dict(os.environ, SWEEP_ROWS=str(rows), SWEEP_CAND=str(cand), SWEEP_DIM=str(dim))
     cmd = [sys.executable, '-m', 'torch.distributed.run', '--nnodes=1', '--nproc-per-node', '2', '--master-addr', '127.0.0.1',
            '--master-port', str(_free_port()), os.path.join(ROOT, 'tools', 'sharded_sweep.py')]

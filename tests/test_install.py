@@ -1,30 +1,33 @@
 """CPU: the drop-in switch patches the reference's registries in place and restores them.
-Runs only where the reference tree is mounted (the build container)."""
+The reference's modules are stood in for by stubs that carry the registry keys and the module-level names
+recorded from it in tests/golden/registry.npz (tests/golden/make_golden.py)."""
 import os
 import sys
 import types
 
-import pytest
-
-REF = '/root/reference'
+import numpy as np
 
 
-@pytest.mark.skipif(not os.path.isdir(REF), reason='reference tree not mounted')
-def test_install_patches_reference_registries():
-    import torch.nn as nn
-    sys.dont_write_bytecode = True
-    added = REF not in sys.path
-    if added:
-        sys.path.insert(0, REF)
-    for name in ['matplotlib', 'matplotlib.pyplot', 'skimage', 'skimage.filters', 'kornia', 'kornia.augmentation']:
-        sys.modules.setdefault(name, types.ModuleType(name))
-    sys.modules['skimage.filters'].gaussian = lambda *a, **k: None
+def _reference_stubs(g):
+    """utils.name_match, experiment.run and the modules whose names install() rebinds, as sys.modules entries."""
+    mods = {n: types.ModuleType(n) for n in ('utils', 'utils.buffer', 'agents', 'experiment', 'utils.name_match',
+                                             'experiment.run', 'agents.base', 'utils.buffer.aser_retrieve',
+                                             'utils.buffer.aser_update')}
+    nm = mods['utils.name_match']
+    for table in ('agents', 'retrieve_methods', 'update_methods'):
+        setattr(nm, table, {k: type('Reference%s' % k, (), {}) for k in g[table].tolist()})
+    mods['experiment.run'].agents = nm.agents if bool(g['run_agents_is_name_match_agents']) else dict(nm.agents)
+    for entry in g['patched'].tolist():
+        mod, attr = entry.split(':')
+        setattr(mods[mod], attr, type('Reference' + attr, (), {}))
+    return mods
 
-    class Identity(nn.Module):
-        def __init__(self, *a, **k):
-            super().__init__()
-    for n in ['RandomResizedCrop', 'RandomHorizontalFlip', 'ColorJitter', 'RandomGrayscale']:
-        setattr(sys.modules['kornia.augmentation'], n, Identity)
+
+def test_install_patches_reference_registries(golden_dir):
+    g = np.load(os.path.join(golden_dir, 'registry.npz'), allow_pickle=False)
+    stubs = _reference_stubs(g)
+    saved = {k: sys.modules[k] for k in stubs if k in sys.modules}
+    sys.modules.update(stubs)
     try:
         import utils.name_match as nm
         import agents.base as base
@@ -45,10 +48,9 @@ def test_install_patches_reference_registries():
         assert (nm.agents['ER'], nm.retrieve_methods['ASER'], nm.update_methods['random'], base.SupConLoss,
                 ar.compute_knn_sv, nm.agents['EWC']) == before
     finally:
-        if added:
-            sys.path.remove(REF)
-        for m in [k for k in sys.modules if k.split('.')[0] in ('utils', 'agents', 'experiment', 'continuum', 'models')]:
-            del sys.modules[m]
+        for k in stubs:
+            sys.modules.pop(k, None)
+        sys.modules.update(saved)
 
 
 def test_host_sampling_logic():
